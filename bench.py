@@ -8,6 +8,7 @@ object / background points) per candidate, plus one NUNOCS forward (8192 points)
 `config`), `value` = candidates scored / second over all ranks.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config K1|K2|K3|K4|K5]
+                    [--dump-outputs DIR]
 
 Default configuration by GPU count (BASELINE.json `configs`):
     --gpus 1 -> K2  nut clutter pile, 20 000-pt scene, 4 096 candidates                       (weak when forced at N > 1)
@@ -17,6 +18,9 @@ Default configuration by GPU count (BASELINE.json `configs`):
                     (adjust_collision_pose off) -> grasp-Q on the survivors; ~1 M candidates over all ranks
 N > 1 is launched by torchrun (one rank per GPU); no data-path collective, one NCCL all-gather of the 48-byte result
 records per pass.  Prints ONE JSON line (rank 0).
+
+--dump-outputs DIR writes what the timed path returned in its last pass as DIR/<name>.npy (see dump_outputs).  The
+inputs are synthetic and seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -68,7 +72,13 @@ def parse_args():
     ap.add_argument("--cpu-sample", type=int, default=192, help="candidates in the CPU-baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-api-leg", action="store_true", help="skip the e2e_api leg (GraspPredicter.predict_batch wall clock)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last timed pass to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.config is None:
         args.config = "K2" if args.gpus == 1 else ("K3" if args.gpus == 2 else "K4")
     return args
@@ -81,6 +91,30 @@ def load_peaks():
         return {"hbm_gbs": d["hbm_gbs"], "bf16_tflops": d["bf16_tflops"],
                 "bf16_tflops_sustained": d.get("bf16_tflops_sustained", d["bf16_tflops"]), "source": "measured"}
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "source": "fallback"}
+
+
+DUMP_MAX_ROWS = 1 << 16
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as <out_dir>/<name>.npy: float64 stays float64, everything else (probabilities, labels, status
+    and offset codes, poses, NOCS coordinates and bins) becomes float32, which holds each of those integer codes exactly.
+    An array with more than DUMP_MAX_ROWS rows keeps a fixed sample of rows (seeded, so the same rows every run for the
+    same length), listed in <name>_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        if a.shape[0] > DUMP_MAX_ROWS:
+            rows = np.sort(np.random.RandomState(0).choice(a.shape[0], DUMP_MAX_ROWS, replace=False))
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+            total += rows.size * 8
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+        total += a.nbytes
+    assert total <= DUMP_MAX_BYTES, f"dumped {total} bytes, more than {DUMP_MAX_BYTES}"
 
 
 class ClockSampler:
@@ -407,20 +441,22 @@ def main():
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
 
     def one_pass():
-        recs, coords = [], None
+        recs, outs = [], []
         for j in jobs:
             d = j["d"]
-            coords, conf, _ = seg.nunocs_dev(d["nun"], 100)
+            coords, conf, bins = seg.nunocs_dev(d["nun"], 100)
+            outs.append({"nunocs_coords": coords, "nunocs_conf": conf, "nunocs_bins": bins})
             if j["B"] == 0:
                 continue
             probs, label = cls.graspq_dev(d["xyz"], d["nrm"], d["pose"], d["ids"], d_mean, d_std)
             st, off, poses = my_cpp.filter_grasp_pose_raw(d["pose32"], eye[None], eye, eye, g["gripper_in_grasp"], True, True,
                                                           so, d["open"], se, d["bg"])
+            outs[-1].update(graspq_probs=probs, graspq_label=label, filter_status=st, filter_offset=off, filter_poses=poses)
             recs.append(pack_records(probs, st, off))
         rec = torch.cat(recs) if len(recs) > 1 else (recs[0] if recs else torch.zeros((0, 12), device=dev))
         if world > 1:
             rec = all_gather_records(rec, per_rank_max * world)     # one ncclAllGather per pass, no host sync before it
-        return rec, coords
+        return rec, outs
 
     def barrier():
         if world > 1:
@@ -445,11 +481,11 @@ def main():
     passes = args.passes_per_step or int(min(128, max(1, round(1200.0 / (float(pass_ms.item()) * max(args.steps, 1))))))
 
     def step_device():
-        rec = coords = None
+        rec = outs = None
         for _ in range(passes):
             flush.fill_(1)                  # evict L2 between timed passes
-            rec, coords = one_pass()
-        return rec, coords
+            rec, outs = one_pass()
+        return rec, outs
 
     for _ in range(max(args.warmup, 3)):
         step_device()
@@ -464,7 +500,7 @@ def main():
     barrier()
     ev0.record()
     for _ in range(args.steps):
-        rec, coords = step_device()
+        rec, outs = step_device()
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
@@ -472,6 +508,10 @@ def main():
     trunk_ms, trunk_n = ctx.profile_read()
     ctx.profile(False)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        prefix = f"rank{rank}_" if world > 1 else ""
+        dump_outputs(args.dump_outputs, {f"{prefix}scene{s}_{k}": v.cpu().numpy()
+                                         for (s, _, _, _), o in zip(assign, outs) for k, v in o.items()})
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -705,11 +745,11 @@ def run_k5(args, rank, world, local, dev):
                                                     None, none_bg)
         keep = torch.nonzero(st == 0).flatten()
         n_keep = int(keep.numel())
-        probs = None
+        outs = {"filter_status": st, "filter_offset": off, "filter_poses": out}
         if n_keep:
             ids = cls.draw_ids_dev(pts.shape[0], args.n_pts, n_keep, seed=1234, first_candidate=0)
-            probs, _ = cls.graspq_dev(d_xyz, d_nrm, p64[keep].contiguous(), ids)
-        return n_keep, probs
+            outs["graspq_probs"], outs["graspq_label"] = cls.graspq_dev(d_xyz, d_nrm, p64[keep].contiguous(), ids)
+        return n_keep, outs
 
     def barrier():
         if world > 1:
@@ -717,15 +757,19 @@ def run_k5(args, rank, world, local, dev):
         torch.cuda.synchronize()
 
     for _ in range(max(min(args.warmup, 3), 1)):
-        n_keep, probs = one_pass()
+        one_pass()
     barrier()
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     for _ in range(steps):
-        n_keep, probs = one_pass()
+        outs = None                     # drop the last pass's outputs first, so that this pass reuses their memory
+        n_keep, outs = one_pass()
     ev1.record()
     barrier()
+    if args.dump_outputs:
+        prefix = f"rank{rank}_" if world > 1 else ""
+        dump_outputs(args.dump_outputs, {prefix + k: v.cpu().numpy() for k, v in outs.items()})
     t = torch.tensor([ev0.elapsed_time(ev1)], dtype=torch.float64, device=dev)
     k = torch.tensor([n_keep], dtype=torch.float64, device=dev)
     if world > 1:

@@ -57,10 +57,12 @@ def main():
     # FP1: 256 -> 3000 points, skip = the normals (3 + 128 -> [128,128,64])
     sdf1 = make_mlp_state_dict([131, 128, 128, 64], seed=16, conv2d=False)
     f0, idx1, w1 = feature_propagation(ref, sdf1, 3, torch.from_numpy(xyz), l1_xyz, torch.from_numpy(nrm), f1)
+    # f0 in full would put the file over 1 MB: keep a fixed, seeded sample of 512 of its N points
+    f0_cols = np.sort(np.random.RandomState(0).choice(N, 512, replace=False))
     out.update(start1=start1.numpy(), start2=start2.numpy(), l1_xyz=l1_xyz.numpy(), l1_pts=l1_pts.numpy(),
                grouped1=grouped1.numpy()[:, :8], l2_xyz=l2_xyz.numpy(), l2_pts=l2_pts.numpy(), l3_pts=l3_pts.numpy(),
-               f2=f2.numpy(), f1=f1.numpy(), idx2=idx2.numpy(), w2=w2.numpy(), f0=f0.numpy(), idx1=idx1.numpy(),
-               w1=w1.numpy())
+               f2=f2.numpy(), f1=f1.numpy(), idx2=idx2.numpy(), w2=w2.numpy(), f0_cols=f0_cols,
+               f0_sample=np.ascontiguousarray(f0.numpy()[:, :, f0_cols]), idx1=idx1.numpy(), w1=w1.numpy())
     np.savez_compressed(os.path.join(HERE, "pn2_modules.npz"), **out)
     print({k: v.shape for k, v in out.items()}, os.path.getsize(os.path.join(HERE, "pn2_modules.npz")))
 

@@ -860,12 +860,11 @@ def test_occupancy_equals_reference_build(cuda, golden_dir, k):
 
 @pytest.mark.parametrize("k", range(2))
 def test_filterGraspPose_with_ik_equals_reference_build(cuda, golden_dir, k):
-    """filter_ik=True through the 20-argument call, the IK hook being the reference's own ikfast solver (oracle/_ref)."""
+    """filter_ik=True through the 20-argument call, the IK hook answering with the reference's own ikfast verdicts
+    (recorded in tests/golden/mycpp_ik.npz)."""
     from catgrasp_b200 import my_cpp
     from catgrasp_b200.sdf import Sdf3D
     from oracle import mycpp_ref
-    if not mycpp_ref.available():
-        pytest.skip("oracle/_ref (reference ikfast build) not present")
     mk = _mk()
     g_ = np.load(os.path.join(golden_dir, "mycpp_filter.npz"))
     S, scale, mode, adjust, fdir = mk.IK_CASES[k]
@@ -877,7 +876,7 @@ def test_filterGraspPose_with_ik_equals_reference_build(cuda, golden_dir, k):
     my_cpp.register_gripper_sdf(g["enclosed"]["V"], g["enclosed"]["F"], se)
     old = my_cpp.DEFAULT_SDF_MODE
     my_cpp.DEFAULT_SDF_MODE = mode
-    my_cpp.set_ik_solver(lambda ee_in_base, upper, lower: mycpp_ref.ik_solution_count(ee_in_base, upper, lower) > 0)
+    my_cpp.set_ik_solver(mk.recorded_ik_solver(golden_dir, k))
     try:
         res = my_cpp.filterGraspPose(list(poses), list(sym), nocs_pose, c2n, cam, ee, g["gripper_in_grasp"], fdir, True, adjust,
                                      list(mk.IK_UPPER), list(mk.IK_LOWER), g["open"]["V"], g["open"]["F"], g["enclosed"]["V"],
