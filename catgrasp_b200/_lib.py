@@ -89,6 +89,12 @@ SIGNATURES = {
     "cg_fps_single_cta_dev": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
     "cg_ball_query_dev": (_i, [_vp, _f, _i, _vp, _vp, _i, _i, _i, _vp]),
     "cg_group_points_dev": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
+    "cg_cloud_create_dev": (_i, [_vp, _vp, _i, C.c_double, C.POINTER(_vp)]),
+    "cg_cloud_destroy": (None, [_vp]),
+    "cg_cloud_nearest_dev": (_i, [_vp, _vp, _i, _vp, _vp]),
+    "cg_cloud_any_within_dev": (_i, [_vp, _vp, _i, C.c_double, _vp]),
+    "cg_cloud_normals_dev": (_i, [_vp, C.c_double, _i, C.POINTER(C.c_double), _vp, _vp]),
+    "cg_voxel_down_sample_dev": (_i, [_vp, _vp, _vp, _i, C.c_double, _vp, _vp, _vp]),
 }
 
 _lib = None

@@ -415,3 +415,49 @@ def make_mlp_state_dict(dims, seed=0, conv2d=True):
         sd[f"mlp_bns.{i}.running_mean"] = rng.normal(0, 0.2, size=(cout,)).astype(np.float32)
         sd[f"mlp_bns.{i}.running_var"] = rng.uniform(0.5, 1.5, size=(cout,)).astype(np.float32)
     return OrderedDict((k, torch.from_numpy(v)) for k, v in sd.items())
+
+
+# camera of the reference's shipped config (config.yml:1-3): 2064 x 1544 pixels
+REF_CAMERA_K = np.array([[2257.7500557850776, 0, 1032], [0, 2257.4882391629421, 772], [0, 0, 1]], dtype=np.float64)
+REF_CAMERA_HW = (1544, 2064)
+
+
+def make_depth_scene(H, W, K, seed=0, floor_z=0.70, n_spheres=3, n_boxes=3):
+    """Ray-cast depth image (H,W) float32 in metres of a bin floor at camera z = floor_z with a few spheres and
+    axis-aligned boxes resting on it, seen by a pinhole camera K at the origin looking along +z.  Curved surfaces,
+    flat faces and occlusion edges at any resolution (up to the reference camera's 2064 x 1544)."""
+    rng = np.random.RandomState(seed)
+    K = np.asarray(K, dtype=np.float64).reshape(3, 3)
+    v, u = np.meshgrid(np.arange(H, dtype=np.float64), np.arange(W, dtype=np.float64), indexing="ij")
+    dx = (u - K[0, 2]) / K[0, 0]                     # ray direction (dx, dy, 1): the hit's depth is its parameter t
+    dy = (v - K[1, 2]) / K[1, 1]
+    depth = np.full((H, W), floor_z)
+    half = 0.6 * floor_z * min(K[0, 2] / K[0, 0], K[1, 2] / K[1, 1])   # objects stay inside the field of view
+    for _ in range(n_spheres):
+        R = rng.uniform(0.012, 0.030)
+        c = np.array([rng.uniform(-half, half), rng.uniform(-half, half), floor_z - R])
+        dd = dx * dx + dy * dy + 1.0
+        b = dx * c[0] + dy * c[1] + c[2]
+        disc = b * b - dd * (c @ c - R * R)
+        hit = disc >= 0
+        t = np.where(hit, (b - np.sqrt(np.where(hit, disc, 0.0))) / dd, np.inf)
+        depth = np.minimum(depth, t)
+    for _ in range(n_boxes):
+        size = rng.uniform(0.015, 0.045, size=3)
+        ctr = np.array([rng.uniform(-half, half), rng.uniform(-half, half)])
+        lo = np.array([ctr[0] - size[0] / 2, ctr[1] - size[1] / 2, floor_z - size[2]])
+        hi = np.array([ctr[0] + size[0] / 2, ctr[1] + size[1] / 2, floor_z])
+        tmin = np.zeros((H, W))
+        tmax = np.full((H, W), np.inf)
+        for d, a in ((dx, 0), (dy, 1), (np.ones((H, W)), 2)):
+            with np.errstate(divide="ignore", invalid="ignore"):
+                t1 = (lo[a] - 0.0) / d
+                t2 = (hi[a] - 0.0) / d
+            inside = (lo[a] <= 0.0) & (0.0 <= hi[a])
+            t1 = np.where(d == 0, np.where(inside, -np.inf, np.inf), t1)
+            t2 = np.where(d == 0, np.where(inside, np.inf, -np.inf), t2)
+            tmin = np.maximum(tmin, np.minimum(t1, t2))
+            tmax = np.minimum(tmax, np.maximum(t1, t2))
+        t = np.where(tmin <= tmax, tmin, np.inf)
+        depth = np.minimum(depth, t)
+    return depth.astype(np.float32)

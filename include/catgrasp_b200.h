@@ -342,6 +342,45 @@ int  cg_three_interp_dev(cg_ctx *ctx, const float *xyz1, const float *xyz2, cons
                          const float *points2, int D2, int B, int N, int S, float *out,
                          int32_t *out_idx, float *out_weight);
 
+/* ---- point-cloud front end (device pointers, float64) ---------------------------------------
+ * Replaces the open3d / scipy.spatial.cKDTree calls that turn a depth scan into the clouds of the grasp
+ * stage: run_grasp_simulation.py:113-139 and :171-175 (compute_candidate_grasp_one_ob), :198-211 and
+ * :245-251 (compute_candidate_grasp), Utils.py:205-213 (correct_pcd_normal_direction) and :482-488
+ * (cloudA_minus_cloudB).  Distances are ((dx*dx + dy*dy) + dz*dz) in float64, no contraction.
+ *
+ * cg_cloud: (N,3) points plus a grid of their OCCUPIED cells (cell edge `cell`, coarse level 8*cell), memory
+ * O(N).  Create copies and sorts the points and synchronises the context stream (it reads the bounding box
+ * and the number of occupied cells); it is the only call that allocates.  Non-finite points or more than
+ * 2^21 cells along an axis: CG_EINVAL.  N = 0 is a valid, empty cloud.                                     */
+typedef struct cg_cloud cg_cloud;
+int  cg_cloud_create_dev(cg_ctx *ctx, const double *pts, int N, double cell, cg_cloud **out);
+void cg_cloud_destroy(cg_cloud *c);
+/* cKDTree.query(q, k=1) (run_grasp_simulation.py:118-119): exact nearest point, out_dist = sqrt(d^2),
+ * out_idx = its index in the create-time points; ties go to the lower index.  An empty cloud or a
+ * non-finite query gives (inf, N), cKDTree's "no neighbour".                                               */
+int  cg_cloud_nearest_dev(cg_cloud *c, const double *q, int Q, double *out_dist, int32_t *out_idx);
+/* out[i] = 1 iff some point lies within distance <= r of q[i]: the `dists <= gripper_diameter/2` crop of
+ * run_grasp_simulation.py:130-133, and cloudA_minus_cloudB (Utils.py:482-488) with the cloud = B, q = A.     */
+int  cg_cloud_any_within_dev(cg_cloud *c, const double *q, int Q, double r, uint8_t *out);
+/* Normals of the cloud's own points (open3d estimate_normals with KDTreeSearchParamHybrid(radius, max_nn),
+ * run_grasp_simulation.py:208-210,247-249) fused with correct_pcd_normal_direction(view_port):
+ * neighbours = the max_nn nearest points with d^2 < radius^2 (the point itself included, ties to the lower
+ * index), covariance from the cumulants, eigenvector of its smallest eigenvalue; (0,0,1) with fewer than 3
+ * neighbours; then n / (|n| + 1e-10), flipped where it points away from view_port.  1 <= max_nn <= 32.
+ * out_nrm (N,3) in the create-time point order.  out_nbr (N, max_nn) int32 or NULL: the neighbour indices in
+ * ascending distance, padded with N (cKDTree.query(k=max_nn, distance_upper_bound=radius) layout).          */
+int  cg_cloud_normals_dev(cg_cloud *c, double radius, int max_nn, const double view_port[3], double *out_nrm,
+                          int32_t *out_nbr);
+/* open3d voxel_down_sample (run_grasp_simulation.py:114,137,173,246): voxel index
+ * floor((p - (min - 0.5*voxel)) / voxel); every output point (and normal, if nrm != NULL) is the sum of its
+ * voxel's inputs IN INPUT ORDER divided by their count (normals are not re-normalised).  Output order is
+ * ascending voxel index (x, then y, then z) -- open3d emits its hash-map order, which cannot be reproduced.
+ * out_pts / out_nrm need room for N rows; *out_count (DEVICE int32) receives the number of voxels.  Reads the
+ * bounding box back (synchronises the stream).  voxel <= 0, non-finite input, or an index range beyond
+ * int32 (open3d: "voxel_size is too small"): CG_EINVAL.                                                     */
+int  cg_voxel_down_sample_dev(cg_ctx *ctx, const double *pts, const double *nrm, int N, double voxel,
+                              double *out_pts, double *out_nrm, int32_t *out_count);
+
 #ifdef __cplusplus
 }
 #endif
