@@ -77,6 +77,17 @@ SIGNATURES = {
                                        _vp, _vp, _vp]),
     "cg_filter_grasp_pose_dev": (_i, [_vp, C.POINTER(FilterParams), _vp, _i, _vp, _i, _vp, _vp, _i, _vp, _vp, _i,
                                       _vp, _vp, _vp]),
+    "cg_mesh_create": (_i, [_vp, _vp, _i, _vp, _i, C.POINTER(_vp)]),
+    "cg_mesh_destroy": (None, [_vp]),
+    "cg_mesh_info": (_i, [_vp, C.POINTER(_i), C.POINTER(_f), C.POINTER(C.c_int64)]),
+    "cg_voxels_create_dev": (_i, [_vp, _vp, _i, _f, C.POINTER(_vp)]),
+    "cg_voxels_destroy": (None, [_vp]),
+    "cg_voxels_count": (_i, [_vp, C.POINTER(_i)]),
+    "cg_voxels_keys_host": (_i, [_vp, _vp]),
+    "cg_filter_grasp_pose_mesh_dev": (_i, [_vp, C.POINTER(FilterParams), _vp, _i, _vp, _i, _vp, _vp, _vp, _vp,
+                                           _vp, _vp, _vp]),
+    "cg_filter_grasp_pose_mesh_host": (_i, [_vp, C.POINTER(FilterParams), _vp, _i, _vp, _i, _vp, _vp, _i, _vp, _vp,
+                                            _i, _f, _vp, _vp, _vp]),
     "cg_occupancy_grid_geometry": (_i, [_vp, _i, _f, C.POINTER(_i), C.POINTER(_f)]),
     "cg_occupancy_from_scan_host": (_i, [_vp, _vp, _i, _f, _vp]),
     "cg_ransac9d_host": (_i, [_vp, _vp, _vp, _i, _vp, _i, C.c_double, _vp, _vp, _vp, _vp, _vp, _vp]),

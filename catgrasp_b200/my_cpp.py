@@ -4,10 +4,12 @@
 (my_cpp/common.h:60) and returns the surviving grasp_in_cam matrices as a list
 of (4,4) float32 arrays.  Differences, all documented in INTEGRATION.md:
 
-* geometry predicate = gripper SDF vs scene points (sdf.py:292-389) instead of
-  FCL mesh-vs-octree; the SDFs of the two gripper meshes must be registered
-  once with :func:`register_gripper_sdf` (the reference loads the same grids
-  from ``gripper*.sdf``, dexnet/grasping/gripper.py:120-129);
+* default geometry predicate = gripper SDF vs scene points (sdf.py:292-389)
+  instead of FCL mesh-vs-octree; the SDFs of the two gripper meshes must be
+  registered once with :func:`register_gripper_sdf` (the reference loads the
+  same grids from ``gripper*.sdf``, dexnet/grasping/gripper.py:120-129).
+  ``COLLISION_PREDICATE = "mesh"`` evaluates the reference's own mesh-vs-voxel
+  test from the meshes alone, with no SDF;
 * survivors come back in deterministic (pose, symmetry) order, not in OpenMP
   thread-arrival order (common.cpp:303-313);
 * ``filter_ik=True`` needs a host IK predicate registered with
@@ -22,6 +24,7 @@ import torch
 from . import _lib
 
 _SDF_REGISTRY = {}
+_MESH_REGISTRY = {}
 _IK_SOLVER = None
 DEFAULT_SDF_MODE = _lib.CG_SDF_TRILINEAR
 # Which geometry predicate filterGraspPose uses for "the posed gripper touches a scene point":
@@ -29,6 +32,8 @@ DEFAULT_SDF_MODE = _lib.CG_SDF_TRILINEAR
 #   "voxel" -- sd < octo_resolution * sqrt(3) / 2: conservative stand-in for the reference's FCL mesh-vs-octomap test
 #              (collision_manager.cpp:93-111), where a point occupies a whole voxel cube of side octo_resolution -- every
 #              cube that can touch the gripper surface has its generating point within half a cube diagonal of it.
+#   "mesh"  -- the reference's own test: the posed gripper mesh touches an occupied voxel cube of side octo_resolution
+#              (collision_manager.cpp:15-111, restated in oracle/mesh_voxel_ref.py); needs no SDF.
 # Measured agreement with a restatement of the mesh-vs-voxel semantic: DESIGN.md, X2.
 COLLISION_PREDICATE = "sdf"
 
@@ -62,6 +67,14 @@ def _sdf_for(vertices, faces):
         raise _lib.CgError("no SDF registered for this gripper mesh: call "
                            "catgrasp_b200.my_cpp.register_gripper_sdf(vertices, faces, Sdf3D) first")
     return _SDF_REGISTRY[key]
+
+
+def _mesh_for(vertices, faces):
+    key = _digest(vertices, faces)
+    if key not in _MESH_REGISTRY:
+        from .mesh import GripperMesh
+        _MESH_REGISTRY[key] = GripperMesh(vertices, faces)
+    return _MESH_REGISTRY[key]
 
 
 def _m16(m):
@@ -119,6 +132,59 @@ def filter_grasp_pose_raw(grasp_poses, symmetry_tfs, nocs_pose, canonical_to_noc
     return status, offset, poses
 
 
+def filter_grasp_pose_mesh_raw(grasp_poses, symmetry_tfs, nocs_pose, canonical_to_nocs, gripper_in_grasp,
+                               filter_approach_dir_face_camera, adjust_collision_pose, mesh_open, open_pts, mesh_enclosed,
+                               enclosed_pts, octo_resolution, split_status=False):
+    """filter_grasp_pose_raw with the mesh-vs-voxel predicate: mesh_* are catgrasp_b200.mesh.GripperMesh handles;
+    open_pts / enclosed_pts are (N,3) points (host arrays or CUDA tensors) or ready catgrasp_b200.mesh.VoxelSet handles
+    at octo_resolution.  CUDA-tensor poses return device tensors, host poses host arrays."""
+    from .mesh import VoxelSet, _check
+    ctx = mesh_open.ctx
+    prm = _lib.FilterParams()
+    prm.nocs_pose = _m16(nocs_pose)
+    prm.canonical_to_nocs = _m16(canonical_to_nocs)
+    prm.gripper_in_grasp = _m16(gripper_in_grasp)
+    prm.filter_approach_dir_face_camera = int(bool(filter_approach_dir_face_camera))
+    prm.adjust_collision_pose = int(bool(adjust_collision_pose))
+    prm.split_coll_status = int(bool(split_status))
+    enc = mesh_enclosed.h if mesh_enclosed is not None else None
+    on_device = isinstance(grasp_poses, torch.Tensor) and grasp_poses.is_cuda
+    if on_device or isinstance(open_pts, VoxelSet) or isinstance(enclosed_pts, VoxelSet):
+        dev = torch.device("cuda", ctx.device)
+        gp = torch.as_tensor(np.asarray(grasp_poses) if not isinstance(grasp_poses, torch.Tensor) else grasp_poses)
+        gp = gp.to(device=dev, dtype=torch.float32).contiguous().reshape(-1, 16)
+        st = torch.as_tensor(np.asarray(symmetry_tfs)).to(device=dev, dtype=torch.float32).contiguous().reshape(-1, 16)
+        vo = open_pts if isinstance(open_pts, VoxelSet) else VoxelSet(open_pts, octo_resolution, ctx=ctx)
+        ve = enclosed_pts if isinstance(enclosed_pts, VoxelSet) else VoxelSet(enclosed_pts, octo_resolution, ctx=ctx)
+        G, S = gp.shape[0], st.shape[0]
+        Q = G * S
+        status = torch.empty((Q,), dtype=torch.uint8, device=dev)
+        offset = torch.empty((Q,), dtype=torch.int8, device=dev)
+        poses = torch.empty((Q, 4, 4), dtype=torch.float32, device=dev)
+        ctx.use_torch_stream()
+        _check(ctx, ctx.lib.cg_filter_grasp_pose_mesh_dev(
+            ctx.h, C.byref(prm), _lib.ptr(gp), G, _lib.ptr(st), S, mesh_open.h, vo.h, enc, ve.h,
+            _lib.ptr(status), _lib.ptr(offset), _lib.ptr(poses)))
+        if on_device:
+            return status, offset, poses
+        return status.cpu().numpy(), offset.cpu().numpy(), poses.cpu().numpy()
+    gp = np.ascontiguousarray(np.asarray(grasp_poses, dtype=np.float64).astype(np.float32)).reshape(-1, 16)
+    st = np.ascontiguousarray(np.asarray(symmetry_tfs, dtype=np.float64).astype(np.float32)).reshape(-1, 16)
+    p1 = np.ascontiguousarray(np.asarray(open_pts, dtype=np.float64).astype(np.float32)).reshape(-1, 3)
+    p2 = np.ascontiguousarray(np.asarray(enclosed_pts, dtype=np.float64).astype(np.float32)).reshape(-1, 3)
+    G, S = gp.shape[0], st.shape[0]
+    Q = G * S
+    status = np.empty((Q,), np.uint8)
+    offset = np.empty((Q,), np.int8)
+    poses = np.empty((Q, 4, 4), np.float32)
+    ctx.use_own_stream()   # blocking host call
+    _check(ctx, ctx.lib.cg_filter_grasp_pose_mesh_host(
+        ctx.h, C.byref(prm), _lib.ptr(gp), G, _lib.ptr(st), S, mesh_open.h, _lib.ptr(p1), p1.shape[0], enc,
+        _lib.ptr(p2), p2.shape[0], C.c_float(float(np.float32(octo_resolution))),
+        _lib.ptr(status), _lib.ptr(offset), _lib.ptr(poses)))
+    return status, offset, poses
+
+
 def _mm4_f32(A, B):
     """(...,4,4) x (...,4,4) in float32 with the accumulation order of the reference build's Eigen fixed-size product
     (sum over k = 0..3, one rounding per multiply and per add; my_cpp is built without FMA, CMakeLists.txt:5-6) --
@@ -158,17 +224,28 @@ def filterGraspPose(grasp_poses, symmetry_tfs, nocs_pose, canonical_to_nocs_tran
         a = np.asarray(a)
         if a.size and (a.ndim != 2 or a.shape[1] != 3):   # collision_manager.cpp:57-61 (reference exits)
             raise ValueError(f"{name} must be (N,3), got {a.shape}")
-    sdf_open = _sdf_for(gripper_vertices, gripper_faces)
-    sdf_encl = _sdf_for(gripper_enclosed_vertices, gripper_enclosed_faces)
+    if COLLISION_PREDICATE == "mesh":
+        mesh_open = _mesh_for(gripper_vertices, gripper_faces)
+        mesh_encl = _mesh_for(gripper_enclosed_vertices, gripper_enclosed_faces)
+    else:
+        sdf_open = _sdf_for(gripper_vertices, gripper_faces)
+        sdf_encl = _sdf_for(gripper_enclosed_vertices, gripper_enclosed_faces)
     if filter_ik and _IK_SOLVER is None:
         raise NotImplementedError("filter_ik=True requires catgrasp_b200.my_cpp.set_ik_solver(fn); "
                                   "the generated ikfast solver is a host stage (INTEGRATION.md)")
-    status, offset, poses = filter_grasp_pose_raw(
-        grasp_poses, symmetry_tfs, nocs_pose, canonical_to_nocs_transform, gripper_in_grasp,
-        filter_approach_dir_face_camera, adjust_collision_pose, sdf_open,
-        np.asarray(gripper_collision_pts).reshape(-1, 3), sdf_encl,
-        np.asarray(gripper_enclosed_collision_pts).reshape(-1, 3),
-        sdf_margin=voxel_margin(octo_resolution) if COLLISION_PREDICATE == "voxel" else 0.0, split_status=bool(verbose))
+    if COLLISION_PREDICATE == "mesh":
+        status, offset, poses = filter_grasp_pose_mesh_raw(
+            grasp_poses, symmetry_tfs, nocs_pose, canonical_to_nocs_transform, gripper_in_grasp,
+            filter_approach_dir_face_camera, adjust_collision_pose, mesh_open,
+            np.asarray(gripper_collision_pts).reshape(-1, 3), mesh_encl,
+            np.asarray(gripper_enclosed_collision_pts).reshape(-1, 3), octo_resolution, split_status=bool(verbose))
+    else:
+        status, offset, poses = filter_grasp_pose_raw(
+            grasp_poses, symmetry_tfs, nocs_pose, canonical_to_nocs_transform, gripper_in_grasp,
+            filter_approach_dir_face_camera, adjust_collision_pose, sdf_open,
+            np.asarray(gripper_collision_pts).reshape(-1, 3), sdf_encl,
+            np.asarray(gripper_enclosed_collision_pts).reshape(-1, 3),
+            sdf_margin=voxel_margin(octo_resolution) if COLLISION_PREDICATE == "voxel" else 0.0, split_status=bool(verbose))
     keep = status == _lib.CG_ST_ACCEPT
     ik_fail = np.zeros(status.shape[0], bool)
     if filter_ik:
@@ -271,18 +348,25 @@ def augmentGraspPoses(R0, selected_point, sphere_pts, inplane_rot_step, hand_dep
 class CollisionManager:
     """my_cpp/collision_manager.h:33-52 (exported by pybind.cpp:13-18, no Python caller): one posed mesh against one
     point set.  The mesh is represented by its registered SDF (see register_gripper_sdf); isAnyCollision() evaluates
-    the same predicate as filterGraspPose for the single transform set with setTransform()."""
+    the same predicate as filterGraspPose for the single transform set with setTransform().  With
+    COLLISION_PREDICATE = "mesh" it is the reference class's own test: the registered mesh against the occupied voxels
+    of the registered points at the registered resolution, and no SDF is needed."""
 
     def __init__(self):
         self._sdf = None
+        self._mesh = None
         self._pts = np.zeros((0, 3), np.float32)
+        self._res = None
         self._pose = np.eye(4, dtype=np.float32)
 
     def registerMesh(self, vertices, faces):
         vertices, faces = np.asarray(vertices), np.asarray(faces)
         if vertices.ndim != 2 or vertices.shape[1] != 3 or faces.ndim != 2 or faces.shape[1] != 3:
             raise ValueError("registerMesh: V,F must be (N,3)")                  # collision_manager.cpp:17-27 (exit(1))
-        self._sdf = _sdf_for(vertices, faces)
+        if COLLISION_PREDICATE == "mesh":
+            self._mesh = _mesh_for(vertices, faces)
+        else:
+            self._sdf = _sdf_for(vertices, faces)
         return 0
 
     def registerPointCloud(self, pts, resolution):
@@ -290,6 +374,7 @@ class CollisionManager:
         if pts.ndim != 2 or pts.shape[1] != 3:
             raise ValueError("registerPointCloud: pts must be (N,3)")            # collision_manager.cpp:57-61
         self._pts = np.ascontiguousarray(pts, dtype=np.float32)
+        self._res = float(np.float32(resolution))
         return 1
 
     def setTransform(self, pose, ob_id):
@@ -299,6 +384,13 @@ class CollisionManager:
         self._pose = pose.astype(np.float32)
 
     def isAnyCollision(self):
+        if COLLISION_PREDICATE == "mesh":
+            if self._mesh is None or self._res is None:
+                raise _lib.CgError("CollisionManager: registerMesh and registerPointCloud first")
+            eye = np.eye(4)
+            st, _, _ = filter_grasp_pose_mesh_raw(self._pose[None], eye[None], eye, eye, eye, False, False, self._mesh,
+                                                  self._pts, None, np.zeros((0, 3), np.float32), self._res)
+            return bool(st[0] == _lib.CG_ST_REJ_COLL)
         if self._sdf is None:
             raise _lib.CgError("CollisionManager: registerMesh first")
         eye = np.eye(4)

@@ -352,6 +352,75 @@ def make_gripper_proxy(res=0.001, pad_cells=5):
     return {"open": build([palm, f1, f2]), "enclosed": build([palm, f1, f2, gap]), "gripper_in_grasp": gig}
 
 
+def _hexa_mesh(C, n):
+    """Convex hexahedron with corners C (8,3) in _box_mesh order, every (planar) quad face split into an n x n grid
+    of 2 n^2 outward-facing triangles."""
+    faces = [(0, 3, 2, 1), (4, 5, 6, 7), (0, 1, 5, 4), (1, 2, 6, 5), (2, 3, 7, 6), (3, 0, 4, 7)]
+    t = np.linspace(0.0, 1.0, n + 1)
+    Vs, Fs, off = [], [], 0
+    for a, b, c, d in faces:
+        u, v = np.meshgrid(t, t, indexing="ij")
+        u, v = u[..., None], v[..., None]
+        P = (1 - u) * (1 - v) * C[a] + u * (1 - v) * C[b] + u * v * C[c] + (1 - u) * v * C[d]
+        Vs.append(P.reshape(-1, 3))
+        i, j = np.meshgrid(np.arange(n), np.arange(n), indexing="ij")
+        p00 = (i * (n + 1) + j).ravel() + off
+        p10, p01, p11 = p00 + (n + 1), p00 + 1, p00 + n + 2
+        Fs.append(np.concatenate([np.stack([p00, p10, p11], 1), np.stack([p00, p11, p01], 1)]))
+        off += (n + 1) ** 2
+    return np.concatenate(Vs), np.concatenate(Fs).astype(np.int32)
+
+
+def _hexa_sdf(p, C):
+    """max over the six face planes of the signed plane distance: the exact sign of a convex hexahedron, exact
+    distance inside and a lower bound outside."""
+    faces = [(0, 3, 2), (4, 5, 6), (0, 1, 5), (1, 2, 6), (2, 3, 7), (3, 0, 4)]
+    out = None
+    for a, b, c in faces:
+        nrm = np.cross(C[b] - C[a], C[c] - C[a])
+        nrm /= np.linalg.norm(nrm)
+        d = (p - C[a]) @ nrm
+        out = d if out is None else np.maximum(out, d)
+    return out
+
+
+def make_dense_gripper_proxy(res=0.001, pad_cells=5, n=24, chamfer=0.004):
+    """make_gripper_proxy's gripper finely triangulated (2 n^2 triangles per face: 20 736 for the open gripper and
+    27 648 with the swept volume at n = 24, about the density of a real Hand-E mesh), with the inner edge of each
+    finger tip chamfered by ``chamfer`` metres at 45 degrees in the x-y plane, so that some faces are not
+    axis-aligned.  Same dictionary layout as make_gripper_proxy; the SDF grids are the signed plane-distance bound of
+    the convex parts (exact sign)."""
+    def box(lo, hi):
+        V, _ = _box_mesh(np.asarray(lo, np.float64), np.asarray(hi, np.float64))
+        return V
+
+    palm = box([-0.040, -0.030, -0.015], [0.0, 0.030, 0.015])
+    f1 = box([0.0, 0.025, -0.010], [0.045, 0.033, 0.010])
+    f2 = box([0.0, -0.033, -0.010], [0.045, -0.025, 0.010])
+    gap = box([0.0, -0.025, -0.010], [0.045, 0.025, 0.010])
+    # tip corners on the inner (closing) side move back along x: corners 1, 5 of f1 (y = 0.025), 2, 6 of f2 (y = -0.025)
+    f1[[1, 5], 0] -= chamfer
+    f2[[2, 6], 0] -= chamfer
+    lo = np.array([-0.040, -0.033, -0.015]) - pad_cells * res
+    hi = np.array([0.045, 0.033, 0.015]) + pad_cells * res
+    dims = np.round((hi - lo) / res).astype(int) + 1
+    gi, gj, gk = np.meshgrid(np.arange(dims[0]), np.arange(dims[1]), np.arange(dims[2]), indexing="ij")
+    P = lo[None, None, None, :] + res * np.stack([gi, gj, gk], -1)
+
+    def build(parts):
+        sd = np.min(np.stack([_hexa_sdf(P, C) for C in parts], 0), 0)
+        Vs, Fs, off = [], [], 0
+        for C in parts:
+            V, F = _hexa_mesh(C, n)
+            Vs.append(V); Fs.append(F + off); off += V.shape[0]
+        return {"V": np.concatenate(Vs), "F": np.concatenate(Fs).astype(np.int32),
+                "sdf": sd.astype(np.float32), "origin": lo.astype(np.float32), "res": np.float32(res)}
+
+    gig = np.eye(4)
+    gig[0, 3] = -0.035
+    return {"open": build([palm, f1, f2]), "enclosed": build([palm, f1, f2, gap]), "gripper_in_grasp": gig}
+
+
 def sample_lattice_nut(n, seed=0, origin=(-0.012, -0.011, 0.70), spacing=0.001):
     """A tilted hex nut snapped to a 1 mm lattice whose largest extent spans exactly LATTICE_LEVELS positions, in the
     camera frame (z ~ 0.7 m): returns (cloud_xyz (n,3) f64, cloud_normal (n,3) f64 with float32-representable values,

@@ -236,6 +236,66 @@ int cg_filter_grasp_pose_dev(cg_ctx *ctx, const cg_filter_params *prm,
                              cg_sdf *sdf_enclosed, const float *enclosed_pts, int P2,
                              uint8_t *out_status, int8_t *out_offset, float *out_poses);
 
+/* ---- collision filter, mesh-vs-voxel predicate ------------------------------
+ * The reference's own geometry test (my_cpp/collision_manager.cpp:15-111: FCL
+ * BVH of the gripper mesh vs an octomap OcTree of the points), restated in
+ * oracle/mesh_voxel_ref.py and computed here bit for bit:
+ *   occupied voxel  = unique key floor(double(x) * (1.0 / res)) per axis with
+ *                     res = double(float32 resolution); keys outside
+ *                     [-32768, 32768) are dropped (octomap coordToKeyChecked);
+ *                     the cube [key*res, (key+1)*res] per axis;
+ *   posed mesh      = float32 gripper_in_cam of cg_filter_grasp_pose_* widened to
+ *                     double, Vc = ((R0*vx + R1*vy) + R2*vz) + t, no contraction;
+ *   collision       = some cube overlaps some posed triangle under the 13-axis
+ *                     separating-axis test in double (touching collides).
+ *
+ * cg_mesh (registerMesh): the (nv,3) float32 vertices and (nf,3) int32 faces in
+ * the gripper frame plus a uniform grid of cubic cells over their bounding box
+ * with CSR lists of the triangles meeting each (closed) cell, built on the host.
+ * Cell-size rule: edge = max(cbrt(box volume / (2 nf)), extent / 1023), where
+ * the box volume uses each extent clamped below at 1e-3 of the largest one; the
+ * edge grows by 1.25x until there are at most max(64, 4 nf) cells and at most
+ * 1024 along an axis.  Memory: 12 nv + 12 nf + 4 (cells + 1) + 4 entries bytes,
+ * with cells <= max(64, 4 nf) and entries = (cell, triangle) incidences.  It
+ * does not depend on any voxel size.  No triangle, a face index outside
+ * [0, nv) or a non-finite vertex: CG_EINVAL.  cg_mesh_info reports the grid.
+ *
+ * cg_voxels (registerPointCloud): the sorted unique keys of (P,3) float32 DEVICE
+ * points.  It synchronises the context stream and is the call that allocates,
+ * so the filter entries stay allocation-free.  P = 0 is a valid, empty set;
+ * a non-finite point or res <= 0: CG_EINVAL.  cg_voxels_keys_host copies the
+ * keys (K,3) int32 to the host in ascending (x, y, z) order.
+ *
+ * cg_filter_grasp_pose_mesh_dev: cg_filter_grasp_pose_dev with the open gripper
+ * mesh tested against vox_open (the object) and the enclosed gripper mesh
+ * against vox_enclosed (the background, may be NULL or empty).  Statuses,
+ * offsets and poses as above, including split_coll_status; prm->sdf_mode and
+ * prm->sdf_margin are ignored.  Both voxel sets must share one resolution.
+ * cg_filter_grasp_pose_mesh_host: the same from HOST points; it builds the two
+ * voxel sets at octo_resolution itself.                                       */
+typedef struct cg_mesh cg_mesh;
+typedef struct cg_voxels cg_voxels;
+int  cg_mesh_create(cg_ctx *ctx, const float *V, int nv, const int32_t *F, int nf, cg_mesh **out);
+void cg_mesh_destroy(cg_mesh *mesh);
+int  cg_mesh_info(const cg_mesh *mesh, int dims[3], float *cell, int64_t *entries);
+int  cg_voxels_create_dev(cg_ctx *ctx, const float *pts, int P, float res, cg_voxels **out);
+void cg_voxels_destroy(cg_voxels *vox);
+int  cg_voxels_count(const cg_voxels *vox, int *out_K);
+int  cg_voxels_keys_host(cg_voxels *vox, int32_t *out_keys);
+int cg_filter_grasp_pose_mesh_dev(cg_ctx *ctx, const cg_filter_params *prm,
+                                  const float *grasp_poses, int G,
+                                  const float *symmetry_tfs, int S,
+                                  cg_mesh *mesh_open, cg_voxels *vox_open,
+                                  cg_mesh *mesh_enclosed, cg_voxels *vox_enclosed,
+                                  uint8_t *out_status, int8_t *out_offset, float *out_poses);
+int cg_filter_grasp_pose_mesh_host(cg_ctx *ctx, const cg_filter_params *prm,
+                                   const float *grasp_poses, int G,
+                                   const float *symmetry_tfs, int S,
+                                   cg_mesh *mesh_open, const float *open_pts, int P1,
+                                   cg_mesh *mesh_enclosed, const float *enclosed_pts, int P2,
+                                   float octo_resolution,
+                                   uint8_t *out_status, int8_t *out_offset, float *out_poses);
+
 /* ---- occupancy / occlusion grid from a depth scan ----------------------------
  * Replaces: my_cpp/common.cpp:324-431 (makeOccupancyGridFromCloudScan; the K
  * argument of the reference is computed with but never influences its output).
